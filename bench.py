@@ -21,7 +21,11 @@ What one run reports (one JSON line):
                     resident in a bm::b200::device_set (upload once), split of the cold step, result compared with bm::aggregator
   cpu_baseline      the reference on 1 thread (bounded sample) and on all cores (whole workload)
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2|c5]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--workload c3|c2|c5] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned to its caller (rank 0's shard) as float64 .npy files, so that two
+builds can be compared output for output on identical (seeded) inputs: per result column kind, popcount, digest (two 32-bit
+halves), GAP run count, the total, and the 2048 result words of a fixed, seeded sample of columns (GAP columns expanded).
 """
 from __future__ import annotations
 
@@ -438,6 +442,32 @@ def run_e2e(args, ctx, dset, device, world, dist, torch, op, g0, g1, flags, tota
             "host_threads": thr, "numa_node": node.value, "check": chk}
 
 
+DUMP_SAMPLE_COLS = 256
+
+
+def dump_outputs(out_dir, bm, res, meta, total_bits):
+    """float64 .npy files of the last timed step's result (exact: every value is an integer below 2^32)."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    kind, pop, dig, nr = meta
+    cols = np.sort(np.random.default_rng(20261017).choice(kind.size, size=min(DUMP_SAMPLE_COLS, kind.size), replace=False))
+    words = np.zeros((cols.size, 2048), np.float64)
+    for i, c in enumerate(cols):
+        k, bits, gap = res.fetch_column(int(c))
+        bv = bm.BVector(1)
+        if k == bm.BLK_BIT:
+            bv.set_bits(0, bits)
+        elif k == bm.BLK_GAP:
+            bv.set_gap(0, gap)
+        elif k == bm.BLK_FULL:
+            bv.set_full(0)
+        words[i] = bv.block_words(0)
+    arrays = {"kind": kind, "popcnt": pop, "digest_lo": dig & np.uint64(0xFFFFFFFF), "digest_hi": dig >> np.uint64(32), "gap_runs": nr,
+              "total_bits": np.array([total_bits], np.uint64), "sample_cols": cols, "sample_words": words}
+    for name, a in arrays.items():
+        np.save(out / f"{name}.npy", np.asarray(a).astype(np.float64))
+
+
 class _StdoutToStderr:
     """Everything libraries print while the bench runs (NCCL's version banner, warnings ...) goes to stderr, so that stdout
     carries exactly ONE line: the JSON result."""
@@ -538,7 +568,10 @@ def _main():
     ap.add_argument("--no-c5", action="store_true", help="skip the extra config-5 shard line that 8-GPU runs carry")
     ap.add_argument("--cpu-cols", type=int, default=256, help="block columns in the 1-thread cpu_baseline sample")
     ap.add_argument("--ref-threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's result arrays to DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
 
     if args.impl == "reference":
@@ -592,6 +625,8 @@ def _main():
 
     total_bits, any_ = res.total()
     kind_r, pop_r, dig_r, nr_r = res.meta()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, bm, res, (kind_r, pop_r, dig_r, nr_r), total_bits)
     res_bytes = int((kind_r == bm.BLK_BIT).sum()) * 8192 + int(2 * (nr_r[kind_r == bm.BLK_GAP].astype(np.int64) + 1).sum())
     # algorithmic bytes (SURVEY 8d): stored source bytes (bit 8192 B, GAP 2*(len+1) B) + result blocks written + 12 B meta per column
     alg_bytes = counts["bit"] * 8192 + gap_words * 2 + res_bytes + n_cols * 12
